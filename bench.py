@@ -18,6 +18,11 @@ at --new-tokens (SURVEY.md section 8d "fixed 128 new tokens").
 
 --workload {all,b1,b8,decode512,enc64,1p7b}: `all` (default) = b1 headline + extras; any other value = b1 headline
 plus only that extra.  --impl reference times only the CPU restatement (the Rust reference cannot be built: no cargo).
+
+--steps K: each timed pass (e2e, then value) runs exactly K steps.
+--dump-outputs DIR: after the timed steps, write what the last one returned to its caller as DIR/ids.npy (float64
+[clips, --new-tokens], -1 past a clip's end; on N > 1 the ids of every rank's clip, as the gather delivers them).
+Weights and clips are seeded, so the same arguments give the same inputs and two builds can be compared file by file.
 """
 from __future__ import annotations
 
@@ -32,6 +37,7 @@ import time
 
 ROOT = os.path.dirname(os.path.abspath(__file__))
 sys.path.insert(0, ROOT)
+sys.dont_write_bytecode = True      # the benchmark may run from a read-only tree and must leave it untouched
 
 CLIP_SECONDS = 30.0
 METRIC = "real-time factor (audio-sec/wall-sec) Qwen3-ASR-0.6B 30s clips"     # identical in both arms
@@ -149,6 +155,16 @@ def cpu_threads_setup():
     return torch.get_num_threads()
 
 
+def dump_outputs(out_dir: str, ids, width: int) -> None:
+    """Token ids per clip as DIR/ids.npy: float64 (every token id is exact), [clips, width], -1 past a clip's end."""
+    import numpy as np
+    a = np.full((len(ids), width), -1.0, dtype=np.float64)
+    for i, row in enumerate(ids):
+        a[i, :len(row)] = row
+    os.makedirs(out_dir, exist_ok=True)
+    np.save(os.path.join(out_dir, "ids.npy"), a)
+
+
 _ORACLE = {}
 
 
@@ -193,7 +209,9 @@ def reference_arm(args, K, W):
         n_tok, extrapolated = 16, True
     for _ in range(max(0, W - 1)):
         cpu_reference_run(n_tok, 1)
-    times, _, _ = cpu_reference_run(n_tok, K)
+    times, last, _ = cpu_reference_run(n_tok, K)
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, [last.ids], args.new_tokens)
     T = sum(times) / K
     per_tok = None
     if extrapolated:
@@ -281,11 +299,15 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--decode", default=None, choices=[None, "mega", "phases"])
     ap.add_argument("--gemm", default=None, choices=[None, "tc", "simt"])
+    ap.add_argument("--dump-outputs", metavar="DIR", default=None,
+                    help="write the ids returned by the last timed step to DIR/ids.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
     rank = int(os.environ.get("RANK", "0"))
     world = int(os.environ.get("WORLD_SIZE", "1"))
     local_rank = int(os.environ.get("LOCAL_RANK", "0"))
-    K, W = max(1, args.steps), max(args.warmup, 3)       # both arms: W >= 3 warm-up steps
+    K, W = args.steps, max(args.warmup, 3)       # both arms: W >= 3 warm-up steps
     config = base_config(world, args.new_tokens)
 
     if args.impl == "reference":
@@ -321,40 +343,45 @@ def main():
     gather = parallel.IdsGather(world, world, args.new_tokens, dev) if dist is not None else None
 
     def one_step():
+        """-> (per-step result, the ids of every clip of the job as the caller receives them)"""
         r = eng.transcribe_ids([clip], max_new_tokens=args.new_tokens)
         if gather is not None:   # the path's only collective: gather of decoded ids (NCCL over NVLink, device buffers)
-            gather(eng)
-        return r
+            return r, gather(eng)
+        return r, r.ids
 
     for _ in range(W):
-        last = one_step()
+        last, _ = one_step()
     # ---- e2e: host buffers in, ids out ----
     sampler = ClockSampler(local_rank)
     if rank == 0:
         sampler.start()
-    barrier()
-    t0 = time.perf_counter()
-    stage = {}
-    launches = 0
-    dec_ms, dec_steps = 0.0, 0
-    for _ in range(K):
-        last = one_step()
-        for k, v in last.stage_ms.items():
-            stage[k] = stage.get(k, 0.0) + v / K
-        launches = last.kernels_launched
-        dec_ms += last.stage_ms["decode"]; dec_steps += last.decode_steps
-    barrier()
-    t_e2e = time.perf_counter() - t0
-    # ---- value: samples resident in HBM ----
-    eng.set_option("resident", "1")
-    barrier()
-    t0 = time.perf_counter()
-    for _ in range(K):
-        last = one_step()
-    barrier()
-    t_val = time.perf_counter() - t0
-    clocks = sampler.stop() if rank == 0 else None
+    try:
+        barrier()
+        t0 = time.perf_counter()
+        stage = {}
+        launches = 0
+        dec_ms, dec_steps = 0.0, 0
+        for _ in range(K):
+            last, _ = one_step()
+            for k, v in last.stage_ms.items():
+                stage[k] = stage.get(k, 0.0) + v / K
+            launches = last.kernels_launched
+            dec_ms += last.stage_ms["decode"]; dec_steps += last.decode_steps
+        barrier()
+        t_e2e = time.perf_counter() - t0
+        # ---- value: samples resident in HBM ----
+        eng.set_option("resident", "1")
+        barrier()
+        t0 = time.perf_counter()
+        for _ in range(K):
+            last, out_ids = one_step()
+        barrier()
+        t_val = time.perf_counter() - t0
+    finally:                # never leave the nvidia-smi sampler running
+        clocks = sampler.stop() if rank == 0 else None
     eng.set_option("resident", "0")
+    if rank == 0 and args.dump_outputs:
+        dump_outputs(args.dump_outputs, out_ids, args.new_tokens)
     if dist is not None:
         tt = torch.tensor([t_e2e, t_val], dtype=torch.float64, device=dev)
         dist.all_reduce(tt, op=dist.ReduceOp.MAX)
